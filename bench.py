@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    (also writes the last timed step's outputs)
 
 A "step" is one whole compaction job over the workload (SURVEY.md 8d / BASELINE.md §3 config 2:
 8-way major compaction, 100 M entries, 32-B DocKey + 256-B value, kNoCompression SSTs). With N>1
@@ -43,6 +44,8 @@ import sys
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -76,8 +79,52 @@ def parse_args():
     ap.add_argument("--c5-timeout", type=float, default=240.0, help="configs[4]: give up (and still print the line) after this many seconds")
     ap.add_argument("--workload", default="config2", choices=["config2", "mvcc"],
                     help="config2 = BASELINE configs[1] (the bench line); mvcc = configs[3] shape (20 versions/key, "
-                         "history cutoff drops 90 %), scaled to --rows entries, for profiles/ only")
-    return ap.parse_args()
+                         "history cutoff drops 90 %%), scaled to --rows entries, for profiles/ only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (counters, KV-stream digest, a "
+                         "fixed sample of the output files) as DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU engine's outputs: it needs --impl ours")
+    return args
+
+
+DUMP_FILE_BYTES = 2 << 20        # bytes sampled per output file: four files as float32 stay well under 64 MB
+DUMP_WINDOW = 4096
+DUMP_COUNTERS = ("num_input_records", "num_output_records", "num_record_drop_hidden", "num_record_drop_obsolete",
+                 "num_record_drop_feed", "total_input_raw_key_bytes", "total_input_raw_value_bytes",
+                 "total_output_raw_key_bytes", "total_output_raw_value_bytes", "num_output_data_blocks",
+                 "output_data_file_size", "output_meta_file_size")
+
+
+def dump_counters(dumps, prefix, stats):
+    dumps[prefix + "_counters"] = np.array([stats[k] for k in DUMP_COUNTERS], dtype=np.float64)
+
+
+def dump_file_sample(dumps, prefix, buf):
+    """A file the caller receives, as float32 bytes: whole when it fits DUMP_FILE_BYTES, else DUMP_WINDOW-byte windows at
+    seeded offsets (the same for the same file size) plus the last window (the footer); the offsets go alongside."""
+    buf = np.asarray(buf, dtype=np.uint8)
+    if buf.size <= DUMP_FILE_BYTES:
+        dumps[prefix] = buf.astype(np.float32)
+        return
+    n = buf.size // DUMP_WINDOW
+    picks = np.random.default_rng(0).choice(n, DUMP_FILE_BYTES // DUMP_WINDOW - 1, replace=False) * DUMP_WINDOW
+    starts = np.unique(np.append(picks, buf.size - DUMP_WINDOW))
+    dumps[prefix] = buf[starts[:, None] + np.arange(DUMP_WINDOW)].astype(np.float32)
+    dumps[prefix + "_offsets"] = starts.astype(np.float64)
+
+
+def write_dumps(out_dir, dumps):
+    if sum(a.nbytes for a in dumps.values()) > 64 << 20:
+        raise ValueError("output dump over 64 MB")
+    if any(a.dtype not in (np.float32, np.float64) for a in dumps.values()):
+        raise ValueError("output dump arrays must be float32 or float64")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in dumps.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -315,9 +362,13 @@ def emit_json_line(line):
         sys.stdout.flush()
 
 
-def resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, verify, steps, warmup, barrier, world, dist, sample_clocks=False):
+def resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, verify, steps, warmup, barrier, world, dist, sample_clocks=False,
+                 read_last=None):
     """`steps` whole jobs with the input files resident in HBM, timed between barriers (CUDA events + wall clock,
-    max over ranks). Returns (total seconds, per-step stats, clocks, host ms per phase)."""
+    max over ranks). Returns (total seconds, per-step stats, clocks, host ms per phase). With `read_last`, the last timed
+    job is not closed inside the timed region: read_last(job) reads its outputs after that region, while the device input
+    files the job reads from are still allocated, and the job is closed after it."""
+    kept = []
     dev_files = []
     for s in ssts:
         v = s.data_view()
@@ -326,7 +377,7 @@ def resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, veri
         dev_files.append(t)
     host_ms = {"create": 0.0, "add_inputs": 0.0, "run": 0.0, "close": 0.0}
 
-    def step():
+    def step(keep=False):
         t0 = time.perf_counter()
         job = pkg.GpuCompactionJob(device=local_rank, verify_checksums=bool(verify), cuda_stream=stream_ptr, **job_kw)
         t1 = time.perf_counter()
@@ -336,7 +387,10 @@ def resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, veri
         st = job.run()
         t3 = time.perf_counter()
         d = st.as_dict()
-        job.close()
+        if keep:
+            kept.append(job)
+        else:
+            job.close()
         t4 = time.perf_counter()
         for k, v in zip(("create", "add_inputs", "run", "close"), (t1 - t0, t2 - t1, t3 - t2, t4 - t3)):
             host_ms[k] += v * 1e3
@@ -353,7 +407,7 @@ def resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, veri
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.perf_counter()
     e0.record()
-    stats = [step() for _ in range(steps)]
+    stats = [step(keep=read_last is not None and i == steps - 1) for i in range(steps)]
     e1.record()
     barrier()
     wall = time.perf_counter() - t0
@@ -362,7 +416,12 @@ def resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, veri
     tt = torch.tensor([step_s], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
-    del dev_files
+    for job in kept:
+        try:
+            read_last(job)
+        finally:
+            job.close()
+    del dev_files             # only now: the jobs read their inputs in place (ybgpu_job_add_input_device)
     return float(tt.item()), stats, clock_info, {k: round(v / steps, 3) for k, v in host_ms.items()}
 
 
@@ -384,7 +443,6 @@ def main():
         run_reference(args, rank, world)
         return
 
-    import numpy as np
     import torch
     import torch.distributed as dist
     pkg = importlib.import_module("yugabyte-db_b200")
@@ -435,8 +493,24 @@ def main():
 
     # ---- HBM-resident arm: checksum verification ON like the reference (verify_checksums_in_compaction = true,
     # rocksdb/util/options.cc:135, db/version_set.cc:3791-3792); the no-verify figure rides along ----
+    dump = args.dump_outputs and rank == 0
+    dumps = {}
+    dump_info = {"dir": args.dump_outputs,
+                 "note": "the last timed resident step's job.close() ran after the timed region (its outputs were read "
+                         "first): compare timings with runs without --dump-outputs only with that in mind"}
+
+    def read_resident(job):
+        d = job.digest()
+        dumps["value_kv_digest"] = np.array([d >> 32, d & 0xffffffff], dtype=np.float64)      # two exact halves
+        data, meta = job.fetch_output()
+        free, total = torch.cuda.mem_get_info()          # inputs, job buffers and the digest's KV stream all live here
+        dump_info["device_gb_in_use_while_reading"] = round((total - free) / 1e9, 1)
+        dump_counters(dumps, "value", job.stats().as_dict())         # output file sizes are known once fetched
+        dump_file_sample(dumps, "value_data", data)
+        dump_file_sample(dumps, "value_meta", meta)
     total_s, stats, clock_info, host_ms = resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, args.verify,
-                                                       args.steps, args.warmup, barrier, world, dist, sample_clocks=True)
+                                                       args.steps, args.warmup, barrier, world, dist, sample_clocks=True,
+                                                       read_last=read_resident if dump else None)
     nv_steps = max(1, min(args.steps, 5))
     nv_s, nv_stats, _, _ = resident_arm(pkg, torch, ssts, handles, local_rank, stream_ptr, job_kw, 0, nv_steps, 1, barrier, world, dist)
     launches = sum(s["gpu_kernel_launches"] for s in stats)
@@ -555,6 +629,10 @@ def main():
         except Exception as ex:
             single["output_check"] = {"error": "%s: %s" % (type(ex).__name__, ex)}
         e2e = dict(single, pinned_inputs=all(ok for _, ok in pinned), verify_checksums=bool(args.verify))
+        if dump and args.subcompactions <= 1:           # the single job is the e2e result
+            dump_counters(dumps, "e2e", res[-1][0])
+            dump_file_sample(dumps, "e2e_data", out_data[:int(res[-1][0]["output_data_file_size"])])
+            dump_file_sample(dumps, "e2e_meta", out_meta[:int(res[-1][0]["output_meta_file_size"])])
         if args.subcompactions > 1:
             files = [(s.meta_view(), s.data_view()) for s in ssts]
 
@@ -599,6 +677,10 @@ def main():
             assert len(off) == st_d["num_output_data_blocks"] and int(off[-1] + sz[-1]) + 5 == data_bytes
             assert st_d["num_input_records"] == n_entries
             one_check = verify_outputs([(meta, out_data[:data_bytes])])
+            if dump:
+                dump_counters(dumps, "e2e", st_d)
+                dump_file_sample(dumps, "e2e_data", out_data[:data_bytes])
+                dump_file_sample(dumps, "e2e_meta", meta)
             e2e = {"value": round(in_bytes * world * args.steps / ot_s / 1e9, 4), "unit": "GB/s", "steps": args.steps,
                    "h2d_bytes_per_step": int(st_d["h2d_bytes"]), "d2h_bytes_per_step": int(st_d["d2h_bytes"]),
                    "ms_per_step": round(ot_s / args.steps * 1e3, 2), "pinned_inputs": all(ok for _, ok in pinned),
@@ -618,6 +700,8 @@ def main():
             if ok:
                 cudart.cudaHostUnregister(v.ctypes.data)
         del out_data, out_meta
+    if dump:
+        write_dumps(args.dump_outputs, dumps)
 
     # ---- BASELINE configs[2] and configs[3] as sub-results (the bench line itself is configs[1]) ----
     extra = {}
@@ -653,7 +737,7 @@ def main():
                     job.close()
                 return sts
             c3_step()
-            c3_steps = 3
+            c3_steps = min(args.steps, 3)
             barrier()
             t0 = time.perf_counter()
             c3_stats = [c3_step() for _ in range(c3_steps)]
@@ -690,7 +774,7 @@ def main():
                 kw4 = dict(job_kw, cutoff_ht=((c4.base_micros + 18 * 1000 + 500) << 12))
                 c4_in = sum(s_.raw_bytes for s_ in s4)
                 c4_entries = sum(s_.num_entries for s_ in s4)
-                c4_steps = 3
+                c4_steps = min(args.steps, 3)
                 c4_s, c4_stats, _, _ = resident_arm(pkg, torch, s4, h4, local_rank, stream_ptr, kw4, args.verify, c4_steps, 1, barrier, world, dist)
                 roof = pipeline_roofline(c4_stats, c4_in, hbm_peak, c4_steps)
                 extra["configs[3]"] = {
@@ -810,6 +894,8 @@ def main():
     }
     if e2e:
         line["e2e"] = e2e
+    if dump:
+        line["dump_outputs"] = dump_info
     if extra:
         line["configs"] = extra
     if not args.no_cpu_baseline:
@@ -848,7 +934,7 @@ def config5_sharded(args, pkg, torch, dist, rank, world, local_rank, job_kw, hbm
     dist.broadcast_object_list(uid, src=0)
     comm = pkg.RangeComm(uid[0], rank, world, local_rank)
     results = []
-    steps = 2
+    steps = min(args.steps, 2)
     dts = []
     for it in range(1 + steps):                      # one warm-up (communicator set-up, allocator) + `steps` timed
         barrier()

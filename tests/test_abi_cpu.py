@@ -32,8 +32,7 @@ def test_exports_every_declared_symbol(pkg):
 
 def test_status_codes_are_the_reference_numbers(pkg):
     """ybgpu_status values must equal yb::Status::Code (util/status_codes.h) because the adapter casts them; the
-    committed table was extracted from the reference header (tests/golden/extract_status_codes.py) and, when the
-    reference tree is present (build container), is re-checked against the header itself."""
+    committed table was extracted from the reference header (tests/golden/extract_status_codes.py)."""
     import json
     tab = json.load(open(os.path.join(ROOT, "tests", "golden", "status_codes_table.json")))["codes"]
     hdr = open(os.path.join(ROOT, "include", "ybgpu_compaction.h")).read()
@@ -49,10 +48,6 @@ def test_status_codes_are_the_reference_numbers(pkg):
         assert tab[name if name != "Ok" else "Ok"] == int(v), name
     for v, name in pkg.STATUS_NAMES.items():
         assert tab["Ok" if name == "OK" else name] == v
-    ref = "/root/reference/src/yb/util/status_codes.h"
-    if os.path.exists(ref):
-        live = {m[0]: int(m[1]) for m in re.findall(r"YB_STATUS_CODE\((\w+),\s*\w+,\s*(\d+),", open(ref).read())}
-        assert live == tab
 
 
 def test_no_cpu_fallback_without_gpu(pkg):
